@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 300 --warmup 10                      # own arm, default workload
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference --steps 5 --warmup 1                 # the reference's CPU path (oracle port)
+    python bench.py --steps 50 --warmup 5 --dump-outputs DIR              # + the last timed step's outputs as DIR/*.npy
 
 Workloads (BASELINE.json configs):
   linear  (default, config 2)  nn::Linear 4096->4096, bf16, batch 4096 per GPU, fwd + bwd (dX, dW, db)
@@ -504,8 +505,9 @@ def run_own(args):
         losses.append(float(loss_pinned[(steps - 1) & 1]))
         return losses
 
-    def measure(name, steps, warmup, full):
-        """resident-loop timing of one workload (+ e2e, eager and sustained legs when `full`)"""
+    def measure(name, steps, warmup, full, dump_dir=None):
+        """resident-loop timing of one workload (+ e2e, eager and sustained legs when `full`); with `dump_dir`, what the
+        last timed step computed is written there before any other leg runs"""
         wl = Workload(env, name)
         spec = wl.spec
         sampler = ClockSampler(local) if full else None
@@ -514,6 +516,8 @@ def run_own(args):
         fn, graphed = wl.runner("res", wl.step_resident, wl.sets[0])
         counter = lambda: dev.launches + (wl.sync.launches if hasattr(wl.sync, "launches") and not graphed else 0)
         ms, stats, host_ms, launches, clocks = timed(fn, steps, warmup, sampler, counter)
+        if dump_dir and rank == 0:
+            dump_outputs(wl, dump_dir, torch, local)
         per_step = ms / steps
         flops_total = spec["flops_per_rank_step"] * world
         out = {"workload": spec["name"], "scaling": spec["scaling"], "steps": steps, "ms_per_step": round(per_step, 5),
@@ -589,7 +593,7 @@ def run_own(args):
 
     # ---- main workload
     W_ = max(args.warmup, 3)
-    main, mx = measure(args.workload, args.steps, W_, full=not args.profile)
+    main, mx = measure(args.workload, args.steps, W_, full=not args.profile, dump_dir=args.dump_outputs)
     wl = mx["wl"]
     if args.profile:
         if rank == 0:
@@ -655,6 +659,40 @@ def run_own(args):
     if world > 1:
         dist.barrier(group=env.host_group)
         dist.destroy_process_group()
+
+
+PARAM_NAMES = {"linear": ["weight", "bias"], "conv": ["weight", "bias"],
+               "mlp": ["linear1_weight", "linear1_bias", "linear2_weight", "linear2_bias", "linear3_weight", "linear3_bias"],
+               "convnet": ["conv1_weight", "conv1_bias", "conv2_weight", "conv2_bias", "linear_weight", "linear_bias"]}
+DUMP_SAMPLE = 1 << 20           # elements kept of a larger output: a fixed, seeded sample of its flat indices
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(wl, out_dir, torch, index):
+    """Write what the step returns to its caller as <out_dir>/<name>.npy (float32): the root's value (the layer output, or
+    the loss), the gradient of every leaf that has one, and the parameters where an optimizer updated them.  The inputs
+    are seeded, so two builds run with the same arguments can be compared output for output."""
+    from neuronika_b200.variable import VarDiff
+    arrays = {"output": wl.live["root"].data_array()}
+    x = wl.sets[0]["x"]
+    if isinstance(x, VarDiff):
+        arrays["input_grad"] = x.grad_array()
+    for name, p in zip(PARAM_NAMES[wl.name], wl.params):
+        arrays[f"{name}_grad"] = p.grad_array()
+        if wl.opt is not None:
+            arrays[name] = p.data_array()
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, arr in arrays.items():
+        t = as_torch(arr, torch, index).reshape(-1)
+        if arr.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(arr.size, DUMP_SAMPLE, replace=False))
+            host = t[torch.from_numpy(idx).to(t.device)].float().cpu().numpy()
+        else:
+            host = t.float().cpu().numpy().reshape(arr.shape)
+        total += host.nbytes
+        np.save(os.path.join(out_dir, f"{name}.npy"), host)
+    assert total <= DUMP_MAX_BYTES, total
 
 
 def exchange_parity(env, wl):
@@ -919,6 +957,9 @@ def main():
     ap.add_argument("--no-graph", dest="graph", action="store_false", help="enqueue every step eagerly (no CUDA graph)")
     ap.add_argument("--profile", action="store_true",
                     help="only the warm-up + timed steps (no e2e / roofline / cpu legs): for ncu launch lists")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs (rank 0) as DIR/<name>.npy, float32; "
+                         f"outputs above {DUMP_SAMPLE} elements as a fixed seeded sample of that many")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)
